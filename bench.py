@@ -2,7 +2,7 @@
 """bench.py — measurement-update throughput of the B200 engine (and, with --impl reference, of the
 reference's own CPU path) on BASELINE.json's configs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one measurement update (the hot path) over one batch: every particle x every sampled
@@ -260,6 +260,7 @@ def run_reference_arm(args):
     s, dda, scaling, P_rank = build_scene(args.workload, 0, 1)
     threads = host_threads()
     unit_pts = n_lik if n_lik else n_beam
+    workload_particles = s["particles"]
     # give every thread enough particles to amortise its start-up: tile the particle set to >= 64 per thread
     need = threads * 64
     if len(s["particles"]) < need:
@@ -272,6 +273,10 @@ def run_reference_arm(args):
     for _ in range(args.steps):
         cpu.measure(sample, s["lik"], s["beam"], s["origins"], n_threads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        # the timed sample's size follows this host's speed; records are per particle, so the workload's own particle
+        # set (untimed) gives the same records for every particle the timed step covered, at a size fixed by the workload
+        dump_outputs(args.dump_outputs, cpu.measure(workload_particles, s["lik"], s["beam"], s["origins"], n_threads=threads))
     value = n_sample * unit_pts * args.steps / dt
     meta["value"] = value
     meta["unit"] = "evals/s"
@@ -295,6 +300,14 @@ def run_reference_arm(args):
     print(json.dumps(line))
 
 
+def dump_outputs(out_dir, recs):
+    """--dump-outputs: every field of the last timed step's records as DIR/<field>.npy (float32 scores, float64
+    counts), so that two builds can be compared output for output on the same seeded inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    for f in recs.dtype.names:
+        np.save(os.path.join(out_dir, f + ".npy"), recs[f].astype(np.float32 if recs[f].dtype.kind == "f" else np.float64))
+
+
 def metric_name(n_lik):
     return "particle x point likelihood evals/s" if n_lik else "particle x ray beam-model evals/s"
 
@@ -313,9 +326,11 @@ class Ctx:
     pass
 
 
-def device_leg(cx, workload, raycaster, steps, warmup, exchange="peer", graph=True, keep_spinning=False, field=False):
+def device_leg(cx, workload, raycaster, steps, warmup, exchange="peer", graph=True, keep_spinning=False, field=False,
+               keep_records=False):
     """Device-resident leg of one workload on every rank: value (CUDA events, max over ranks), per-model kernel
-    times, counted roofline.  Returns (result dict, live objects for the e2e leg)."""
+    times, counted roofline.  Returns (result dict, live objects for the e2e leg).  keep_records: live["last_records"]
+    holds the records of the last timed step of the headline protocol, as the caller of measure_device receives them."""
     import torch
     import torch.distributed as dist
     from mcl_3dl_b200 import engine, sharding
@@ -435,10 +450,21 @@ def device_leg(cx, workload, raycaster, steps, warmup, exchange="peer", graph=Tr
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item()), per
 
+    def records():
+        """The records the step left on the device: this rank's array, or every rank's after the exchange."""
+        buf = d_all if world > 1 else d_out
+        if peer:
+            ptr, _ = eng.exchange_current(torch.cuda.current_stream().cuda_stream)
+            cai = {"shape": (world * P_rank * 24,), "typestr": "|u1", "data": (ptr, False), "version": 3}
+            buf = torch.as_tensor(type("DeviceBytes", (), {"__cuda_array_interface__": cai})(), device=dev)
+        torch.cuda.synchronize()
+        return np.frombuffer(buf.cpu().numpy().tobytes(), dtype=synth.RESULT).copy()
+
     for _ in range(warmup):
         step()
     barrier()
     total_ms, per_step = timed(step, steps)
+    last_records = records() if keep_records else None
     if keep_spinning:
         # the timed region lasts a few milliseconds, shorter than one nvidia-smi period: keep the same step running
         # (untimed, same count on every rank) for ~0.5 s so that the clock record holds samples taken under this load
@@ -502,6 +528,8 @@ def device_leg(cx, workload, raycaster, steps, warmup, exchange="peer", graph=Tr
                 g_rot.replay()
             barrier()
             official = replay_ms(g_rot)                       # the timed region: exactly `steps` steps
+            if keep_records and L2_MODE == "rotate":
+                last_records = records()
             repeats = [replay_ms(g_rot) for _ in range(4)]
             g_same = capture(lambda i: 0)                     # comparison: every step on the same inputs (L2-warm)
             g_same.replay()
@@ -629,7 +657,8 @@ def device_leg(cx, workload, raycaster, steps, warmup, exchange="peer", graph=Tr
     res["map"] = {"nn_grid": list(info.nn_dims), "dda_grid": list(info.dda_dims), "device_bytes": int(info.device_bytes),
                   "build_ms": round(info.build_ms, 3)}
     live = {"eng": eng, "scene": s, "dda": dda, "P_rank": P_rank, "d_out": d_out, "plain_measure": plain_measure,
-            "n_lik": n_lik, "n_beam": n_beam, "spread": spread, "P": P, "scaling": scaling, "unit_pts": unit_pts}
+            "n_lik": n_lik, "n_beam": n_beam, "spread": spread, "P": P, "scaling": scaling, "unit_pts": unit_pts,
+            "last_records": last_records}
     return res, live
 
 
@@ -831,7 +860,11 @@ def main():
     ap.add_argument("--raycaster", default="dda", choices=["dda", "kd"],
                     help="beam raycaster: RaycastUsingDDA (north_star) or RaycastUsingKDTree (the node's default)")
     ap.add_argument("--spread", action="store_true", help="spread (global-localisation style) particles: the HBM-bound variant")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the records of the last timed step (one .npy per field, seeded inputs) into DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     global FORCE_SPREAD, USE_DDA, L2_MODE
     L2_MODE = "flush" if args.no_graph else args.l2
@@ -866,10 +899,13 @@ def main():
     if rank == 0:
         clocks.start()
     graph = not args.no_graph
-    res, live = device_leg(cx, args.workload, args.raycaster, args.steps, args.warmup, args.exchange, graph, keep_spinning=True)
+    res, live = device_leg(cx, args.workload, args.raycaster, args.steps, args.warmup, args.exchange, graph, keep_spinning=True,
+                           keep_records=bool(args.dump_outputs))
     e2e = e2e_leg(cx, args.workload, args.raycaster, args.steps, live)
     clk = clocks.stop() if rank == 0 else None
     n_lik, n_beam, P_rank, s = live["n_lik"], live["n_beam"], live["P_rank"], live["scene"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, live["last_records"])
 
     # ---- sanity: device-resident records == host-path records (N == 1; at N > 1 the e2e leg checked shard 0)
     if rank == 0 and world == 1 and n_lik and n_beam:
@@ -899,12 +935,12 @@ def main():
     out_host = live.get("out_host")
     del live
 
-    # ---- driver-run secondaries (fewer steps; no CPU leg): what north_star names besides the primary metric
+    # ---- driver-run secondaries (no CPU leg): what north_star names besides the primary metric
     secondaries = {}
     if not args.no_secondaries and args.workload == "c2" and not args.spread:
         sec = ([("c5", "c5", "dda")] if world > 1 else
                [("c3", "c3", "dda"), ("c3_kd", "c3", "kd"), ("c5", "c5", "dda"), ("c5_field", "c5", "dda")])
-        k = max(10, min(args.steps, 30))
+        k = args.steps
         for name, wl, caster in sec:
             try:
                 r2, live2 = device_leg(cx, wl, caster, k, 3, args.exchange, graph, field=name.endswith("_field"))
@@ -923,7 +959,7 @@ def main():
                 secondaries[name] = {"error": "%s: %s" % (type(exc).__name__, exc)}
         if world == 1:
             try:
-                secondaries["c5_resident"] = resident_leg(cx, "c5", max(10, min(args.steps, 30)))
+                secondaries["c5_resident"] = resident_leg(cx, "c5", args.steps)
             except Exception as exc:
                 secondaries["c5_resident"] = {"error": "%s: %s" % (type(exc).__name__, exc)}
         USE_DDA = args.raycaster == "dda"

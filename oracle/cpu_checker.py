@@ -107,13 +107,16 @@ def lib_path(kind):
         return os.path.join(HERE, "libmcl3dl_oracle.so")
     if kind == "reference":
         return os.path.join(HERE, "_ref", "libmcl3dl_ref.so")
+    if kind == "adapter":
+        return os.path.join(HERE, "_ref", "adapter_parity_test")
     raise ValueError(kind)
 
 
 def build(kind="port", quiet=True):
-    """Compile the checker if its .so is missing (make in oracle/)."""
+    """Compile the checker if its .so is missing (make in oracle/).  kind="adapter": the host C++ adapter's parity
+    program, which links the engine library (build that first)."""
     path = lib_path(kind)
-    target = [] if kind == "port" else ["ref"]
+    target = {"port": [], "reference": ["ref"], "adapter": ["adapter"]}[kind]
     if kind == "reference" and not os.path.isdir("/root/reference/include/mcl_3dl"):
         return os.path.exists(path)
     r = subprocess.run(["make", "-C", HERE] + target, capture_output=quiet, text=True)

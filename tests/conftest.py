@@ -42,15 +42,16 @@ def port():
 
 @pytest.fixture(scope="session")
 def reference():
-    """The reference's own sources compiled against shims (oracle/_ref); skip where unavailable."""
+    """The original project's own CPU models, as answers recorded from its build (tests/recorded_reference.py).
+    MCL3DL_RECORD_REFERENCE=1 records them afresh from the live build in oracle/_ref (tests/golden/make_golden.py)."""
+    from recorded_reference import recording, replaying
+    if not os.environ.get("MCL3DL_RECORD_REFERENCE"):
+        yield replaying()
+        return
     from oracle import cpu_checker as cc
-    try:
-        ok = cc.build("reference")
-    except RuntimeError:
-        ok = cc.available("reference")
-    if not ok:
-        pytest.skip("oracle/_ref not built and /root/reference absent")
-    return cc.CpuChecker("reference")
+    ref, store = recording(cc.CpuChecker("reference"))
+    yield ref
+    store.save()
 
 
 def golden(name):

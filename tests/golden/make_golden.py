@@ -1,7 +1,8 @@
 """Regenerate tests/golden/*.npz by running the REFERENCE's own sources (oracle/_ref).
 
 Only runnable in the development container (needs /root/reference to build oracle/_ref).
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py           # the fixtures below
+    python tests/golden/make_golden.py --calls   # reference_calls.npz
 The committed .npz files hold inputs AND the reference outputs, so the GPU box (which has no
 /root/reference) can check both the port oracle and the CUDA engine against them.
 
@@ -14,8 +15,12 @@ Fixtures
                              synthetic room scenes (mcl_3dl_b200.synth) -> per-particle records + per-ray status.
   chunked_radius_search.npz  random ChunkedKdtree::radiusSearch queries (ids + d2), incl. chunk borders.
   transform.npz              State6DOF::transform of random points by random (non-unit) quaternions.
+  reference_calls.npz        the reference's answers to every call of the tests that compare the port with it call by
+                             call (the `reference` fixture, tests/recorded_reference.py): those tests run once against
+                             the live build and record what it returned.
 """
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -146,8 +151,18 @@ def gen_transform(ref):
     print("transform ok")
 
 
+def gen_calls():
+    env = dict(os.environ, MCL3DL_RECORD_REFERENCE="1")
+    tests = [os.path.join(ROOT, "tests", t) for t in ("test_oracle_golden.py", "test_oracle_properties.py")]
+    subprocess.run([sys.executable, "-m", "pytest", "-q", "-p", "no:cacheprovider", "-k", "reference"] + tests,
+                   env=env, check=True)
+
+
 if __name__ == "__main__":
     assert cc.build("reference"), "oracle/_ref cannot be built here (no /root/reference)"
+    if "--calls" in sys.argv:
+        gen_calls()
+        sys.exit(0)
     ref = cc.CpuChecker("reference")
     gen_beam_likelihood(ref)
     gen_room(ref, "room_iso", (1, 1, 1), False, seed=100)

@@ -5,8 +5,8 @@ Three anchors, all CPU-only:
      test_chunked_kdtree.cpp, test_quat.cpp, test_pf.cpp (cited per test);
   2. tests/golden/*.npz — outputs of the reference's own sources (oracle/_ref), committed with the
      generating script tests/golden/make_golden.py;
-  3. when oracle/_ref is present (dev container, or shipped prebuilt to the GPU box): port == reference
-     bit-for-bit on fresh random scenes.
+  3. port == reference bit-for-bit on seeded random scenes, against the reference build's answers recorded in
+     tests/golden/reference_calls.npz (the `reference` fixture, tests/recorded_reference.py).
 """
 import math
 
@@ -356,7 +356,7 @@ def test_golden_transform(port):
         assert np.array_equal(port.quat_rotate(q, g["v"][i]), g["rotated_raw"][i])
 
 
-# ---------------------------------------------------------------- live cross-check with oracle/_ref
+# ---------------------------------------------------------------- cross-check with the recorded reference build
 @pytest.mark.parametrize("seed,w,spread,use_dda", [(1, (1, 1, 1), False, True), (2, (1, 1, 5), False, True),
                                                    (3, (1, 1, 5), True, True), (4, (2, 0.5, 3), False, True),
                                                    (5, (1, 1, 1), False, False), (6, (1, 1, 5), False, False),

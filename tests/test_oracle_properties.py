@@ -1,13 +1,29 @@
 """Property tests (hypothesis): the repo-owned oracle equals the reference's own sources bit for bit on random
 small worlds — DDA walks (every visited voxel), KD-tree walks (positions, sin_angle_), radius search, per-ray
-BeamStatus and per-particle records.  Needs oracle/_ref (prebuilt in the development container)."""
+BeamStatus and per-particle records.  The reference's answers are recorded (tests/recorded_reference.py), so every
+test runs a fixed, seeded set of examples drawn from its strategies' domain rather than fresh draws."""
 import numpy as np
-from hypothesis import HealthCheck, given, settings
+from hypothesis import HealthCheck, Phase, example, given, settings
 from hypothesis import strategies as st
 
 from oracle import cpu_checker as cc
 
-SET = dict(max_examples=60, deadline=None, suppress_health_check=[HealthCheck.function_scoped_fixture])
+
+def recorded_examples(count, **domain):
+    """@given over `domain` (name -> (lo, hi) integer range or list of choices), run as `count` explicit examples drawn
+    from it with a fixed seed and nothing else: the reference's answers exist for exactly these inputs."""
+    rng = np.random.default_rng(count * 7919 + len(domain))
+    cases = [{k: (int(rng.integers(v[0], v[1] + 1)) if isinstance(v, tuple) else v[int(rng.integers(len(v)))])
+              for k, v in domain.items()} for _ in range(count)]
+    strategies = {k: st.integers(*v) if isinstance(v, tuple) else st.sampled_from(v) for k, v in domain.items()}
+
+    def deco(f):
+        f = given(**strategies)(f)
+        for c in cases:
+            f = example(**c)(f)
+        return settings(phases=[Phase.explicit], deadline=None,
+                        suppress_health_check=[HealthCheck.function_scoped_fixture])(f)
+    return deco
 
 
 def world(seed, n):
@@ -28,9 +44,7 @@ def world(seed, n):
     return cc.points(pts, lab), rng
 
 
-@settings(**SET)
-@given(seed=st.integers(0, 10_000), n=st.integers(4, 120), grid=st.sampled_from([0.05, 0.1, 0.2, 0.37]),
-       tol=st.sampled_from([0.0, 0.1, 0.3]))
+@recorded_examples(60, seed=(0, 10_000), n=(4, 120), grid=[0.05, 0.1, 0.2, 0.37], tol=[0.0, 0.1, 0.3])
 def test_dda_walk_matches_reference(port, reference, seed, n, grid, tol):
     m, rng = world(seed, n)
     ctor = [0.1, 0.1, 0.1, grid, 0.25 * np.pi / 180.0 if seed % 2 else 0.5, tol]
@@ -44,8 +58,7 @@ def test_dda_walk_matches_reference(port, reference, seed, n, grid, tol):
         assert np.array_equal(a[0], p[0]) and np.array_equal(a[1], p[1]) and a[2] == p[2]
 
 
-@settings(**SET)
-@given(seed=st.integers(0, 10_000), n=st.integers(4, 120), hit=st.sampled_from([0.0, 0.17, 0.3]))
+@recorded_examples(60, seed=(0, 10_000), n=(4, 120), hit=[0.0, 0.17, 0.3])
 def test_kd_walk_matches_reference(port, reference, seed, n, hit):
     m, rng = world(seed, n)
     ctor = [0.1, 0.1 if seed % 2 else 0.05, 0.1, hit]
@@ -58,9 +71,7 @@ def test_kd_walk_matches_reference(port, reference, seed, n, hit):
         assert a[3] == p[3]
 
 
-@settings(max_examples=25, deadline=None, suppress_health_check=[HealthCheck.function_scoped_fixture])
-@given(seed=st.integers(0, 10_000), n=st.integers(20, 400), use_dda=st.booleans(),
-       w=st.sampled_from([(1, 1, 1), (1, 1, 5), (2, 1, 3)]))
+@recorded_examples(25, seed=(0, 10_000), n=(20, 400), use_dda=[False, True], w=[(1, 1, 1), (1, 1, 5), (2, 1, 3)])
 def test_records_match_reference(port, reference, seed, n, use_dda, w):
     m, rng = world(seed, n)
     lik = cc.lik_params(dist_weight=w, match_dist_min=0.2 if seed % 2 else 0.35)
